@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — headline benchmark of the Module A Krylov hot path (contract: see the task statement / DESIGN.md §6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n 256]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n 256] [--dump-outputs DIR]
 
 Metric (BASELINE.json): CG iterations/s, fp64, 7-point Poisson n^3 (n=256 on one GPU), b = ones, tol = 1e-8.
 A "step" is ONE full CG solve of that system (611 iterations) made through the reference-facing API
@@ -33,6 +33,11 @@ BASELINE configs[4] geometry: 2n x 2n planes, n/4 planes per GPU, so N = 8 is ex
 N * global iterations/s.  Every N > 1 line carries a `parity` object (a full tol=1e-8 solve of the global system
 checked by an independent residual computed with torch from the all-gathered x; mismatch => exit code 3) and
 `extra.strong` (the SAME (2n)^3 system split over the N GPUs).
+
+--dump-outputs DIR (one process: N = 1 or --impl reference) writes what the last timed step returned to its caller as
+float64 .npy files, so that two builds can be compared output for output on identical inputs: x.npy and info.npy.  An x
+of more than DUMP_MAX_ENTRIES entries is replaced by a fixed sample of its rows (seed 0), x.npy then holds x at the rows
+listed in x_index.npy.
 """
 import argparse
 import json
@@ -60,6 +65,7 @@ KERNEL_NAMES = {0: "bk_spmv_stream_kernel", 1: "bk_spmv_vector_kernel", 2: "bk_s
 METRIC = "cg_iterations_per_second"
 UNIT = "it/s"
 FALLBACK_HBM_GBS = 6650.0
+DUMP_MAX_ENTRIES = 1 << 21      # 16 MB of sampled x + 16 MB of its row indices: at most 32 MB per dump
 
 
 def measured_peak():
@@ -70,6 +76,22 @@ def measured_peak():
         except Exception:
             pass
     return FALLBACK_HBM_GBS, "fallback"
+
+
+def dump_outputs(out_dir, x, info):
+    """Write the solve's result (x, info) as float64 .npy files under out_dir (see the module docstring)."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    x = x.detach().to("cpu", torch.float64).reshape(-1)
+    if x.numel() > DUMP_MAX_ENTRIES:
+        idx = torch.randperm(x.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ENTRIES].sort().values
+        np.save(out / "x_index.npy", idx.to(torch.float64).numpy())
+        x = x[idx]
+    else:
+        (out / "x_index.npy").unlink(missing_ok=True)     # left by an earlier, sampled dump into the same directory
+    np.save(out / "x.npy", x.numpy())
+    np.save(out / "info.npy", np.array(info, dtype=np.float64))
 
 
 def workload_config(n, tol):
@@ -188,9 +210,11 @@ def run_reference(args, rank, world):
     t0 = time.perf_counter()
     its = 0
     for _ in range(args.steps):
-        _x, _i, st = orc.cg(A, b, tol=0.0, atol=0.0, maxiter=window)
+        x, info, st = orc.cg(A, b, tol=0.0, atol=0.0, maxiter=window)
         its += st["iterations"]
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, x, info)
     value = its / dt
     sample = (f"{args.steps} x fixed window of {window} CG iterations (tol=0, same recurrences as the tol={args.tol:g} "
               f"solve, which takes 611) on P3D-{n}, torch CPU, {cores} threads, {dt:.0f} s")
@@ -354,6 +378,8 @@ def run_single(args):
         ev1.record()
         torch.cuda.synchronize()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, x, info)
     value = its / (ms * 1e-3)
     last = dict(res)
     m = _native.register_matrix(A)
@@ -658,7 +684,11 @@ def main():
     ap.add_argument("--dist-window", type=int, default=200, help="N>1: CG iterations per timed step")
     ap.add_argument("--strong", action="store_true", help="N>1: make the strong-scaling split the headline value")
     ap.add_argument("--ref-window", type=int, default=100, help="--impl reference: CG iterations per step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's solution x and info as float64 .npy files to DIR (one process)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
@@ -667,6 +697,8 @@ def main():
     if world > 1 or args.gpus > 1 or args.strong or os.environ.get("BK_BENCH_FORCE_DIST"):  # env: 1-rank run of the multi-GPU path
         if "RANK" not in os.environ:
             raise SystemExit("launch multi-GPU runs with torch.distributed.run (one rank per GPU)")
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the result of one process: use it with --gpus 1 or --impl reference")
         run_dist(args, rank, world)
     else:
         run_single(args)

@@ -53,8 +53,8 @@ def main():
     from pytorch_sparse_solver import problems           # our generators (product code; no solver involved)
     from oracle import krylov_oracle as orc
     GOLD.mkdir(parents=True, exist_ok=True)
-    manifest = {"torch": torch.__version__, "generated": time.strftime("%Y-%m-%dT%H:%M:%SZ", time.gmtime()),
-                "cases": {}}
+    manifest = {"torch": torch.__version__, "torch_threads": torch.get_num_threads(),
+                "generated": time.strftime("%Y-%m-%dT%H:%M:%SZ", time.gmtime()), "cases": {}}
 
     def run_ref(kind, A, b, x0=None, **kw):
         calls = {"n": 0}

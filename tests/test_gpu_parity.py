@@ -1476,3 +1476,37 @@ def test_full_size_spmv_all_stagings_bitwise(kind):
     _native.clear_cache()
     m = _native.register_matrix(A)
     assert torch.equal(m.spmv(2.0 * x), 2.0 * outs["k5"][0])
+
+
+def test_bench_dump_outputs_match_oracle(tmp_path):
+    """`bench.py --dump-outputs` writes the solution of the timed call (module_a.cg on the GPU), the same bits from run to
+    run, and it agrees with the oracle's solve of the same system; --steps sets the number of timed solves."""
+    import json
+    import subprocess
+    import sys
+    import numpy as np
+    from conftest import ROOT
+    from oracle import krylov_oracle as orc
+    from pytorch_sparse_solver import problems
+
+    def run(out, steps):
+        cmd = [sys.executable, str(ROOT / "bench.py"), "--gpus", "1", "--n", "32", "--steps", str(steps), "--warmup", "1",
+               "--no-e2e", "--no-cpu", "--no-extra", "--dump-outputs", str(out)]
+        p = subprocess.run(cmd, cwd=str(ROOT), capture_output=True, text=True, timeout=600)
+        assert p.returncode == 0, p.stderr[-4000:]
+        (line,) = [json.loads(ln) for ln in p.stdout.splitlines() if ln.startswith("{")]
+        assert line["steps"] == steps and line["details"]["info"] == 0
+        return line, {f.stem: np.load(f) for f in sorted(out.iterdir())}
+
+    line2, a = run(tmp_path / "a", 2)
+    line4, b = run(tmp_path / "b", 4)
+    its = line2["details"]["iterations_per_solve"]
+    assert line4["details"]["iterations_per_solve"] == its
+    assert abs(line2["ms_per_step"] * 2 * line2["value"] * 1e-3 - 2 * its) <= 1e-6 * its
+    assert abs(line4["ms_per_step"] * 4 * line4["value"] * 1e-3 - 4 * its) <= 1e-6 * its
+    assert sorted(a) == ["info", "x"] and all(v.dtype == np.float64 for v in a.values())
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    A = problems.poisson3d_csr(32)
+    x_ref, info_ref, _ = orc.cg(A, torch.ones(A.shape[0], dtype=torch.float64), tol=1e-8)
+    assert float(a["info"]) == info_ref == 0
+    assert rel_diff(torch.from_numpy(a["x"]), x_ref) <= FP64_TOL

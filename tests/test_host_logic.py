@@ -248,3 +248,48 @@ def test_bench_reference_arm_contract_on_cpu():
     (line2,) = run({"RANK": "0", "WORLD_SIZE": "2", "LOCAL_RANK": "0"}, 2)
     assert line2["n_gpus"] == 2 and "row-partitioned over 2 GPUs" in line2["config"]["workload"]
     assert run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"}, 2) == []
+
+
+def test_bench_dump_outputs_reference_arm(tmp_path):
+    """`--dump-outputs DIR` writes the last timed step's (x, info) as float64 arrays; the same arguments give the same
+    files, and x is what the timed call computes."""
+    import json
+    import subprocess
+    import sys
+    import numpy as np
+    from oracle import krylov_oracle as orc
+    from pytorch_sparse_solver import problems
+
+    def run(out, steps):
+        cmd = [sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--n", "10", "--steps", str(steps),
+               "--warmup", "1", "--ref-window", "7", "--dump-outputs", str(out)]
+        p = subprocess.run(cmd, cwd=str(ROOT), capture_output=True, text=True, timeout=300)
+        assert p.returncode == 0, p.stderr[-2000:]
+        (line,) = [json.loads(ln) for ln in p.stdout.splitlines() if ln.startswith("{")]
+        assert line["steps"] == steps
+        return {f.stem: np.load(f) for f in sorted(out.iterdir())}
+
+    a, b = run(tmp_path / "a", 2), run(tmp_path / "b", 3)
+    assert sorted(a) == ["info", "x"] and all(v.dtype == np.float64 for v in a.values())
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    A = problems.poisson3d_csr(10)
+    x, info, _ = orc.cg(A, torch.ones(A.shape[0], dtype=torch.float64), tol=0.0, atol=0.0, maxiter=7)
+    assert np.array_equal(a["x"], x.numpy()) and float(a["info"]) == info
+
+
+def test_bench_dump_outputs_sample(tmp_path, monkeypatch):
+    """An x larger than DUMP_MAX_ENTRIES is stored as a fixed sample of rows plus the sampled row indices."""
+    import numpy as np
+    import bench
+    monkeypatch.setattr(bench, "DUMP_MAX_ENTRIES", 100)
+    x = torch.randn(1000, dtype=torch.float64)
+    a, b = tmp_path / "a", tmp_path / "b"
+    bench.dump_outputs(a, x, 0)
+    bench.dump_outputs(b, x, 0)
+    idx, xs = np.load(a / "x_index.npy"), np.load(a / "x.npy")
+    assert idx.dtype == xs.dtype == np.float64 and idx.shape == xs.shape == (100,)
+    assert np.all(np.diff(idx) > 0) and np.array_equal(xs, x.numpy()[idx.astype(np.int64)])
+    assert np.array_equal(idx, np.load(b / "x_index.npy"))
+    bench.dump_outputs(a, x[:50].float(), 1)
+    assert sorted(f.name for f in a.iterdir()) == ["info.npy", "x.npy"]
+    assert np.load(a / "x.npy").dtype == np.float64 and float(np.load(a / "info.npy")) == 1.0

@@ -11,6 +11,16 @@ from oracle import krylov_oracle as orc
 SLOW = {"gmres_ldc100_step0_incremental", "gmres_ldc100_step1_batched"}
 
 
+@pytest.fixture(autouse=True)
+def golden_threads(manifest):
+    """torch's CPU reductions split their sums by the number of threads, so the oracle reproduces the reference's bits
+    only with the thread count the goldens were pinned with, whatever the cores of the machine running the tests."""
+    saved = torch.get_num_threads()
+    torch.set_num_threads(manifest["torch_threads"])
+    yield
+    torch.set_num_threads(saved)
+
+
 def _case_names():
     import json
     from conftest import GOLD
