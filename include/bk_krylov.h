@@ -37,6 +37,7 @@ extern "C" {
 typedef struct bk_handle bk_handle; /* per-device context: scratch, workspaces, graph cache */
 typedef struct bk_csr bk_csr;       /* a registered CSR matrix + its kernel plan */
 typedef struct bk_dist bk_dist;     /* row-partitioned (multi-GPU) matrix + halo plan */
+typedef struct bk_sgs bk_sgs;       /* multicolor symmetric Gauss-Seidel preconditioner of a registered matrix */
 
 enum bk_error {
   BK_OK = 0,
@@ -237,6 +238,33 @@ int bk_bicgstab_jacobi(bk_handle* h, const bk_csr* A, const void* diag, const vo
 int bk_gmres_jacobi(bk_handle* h, const bk_csr* A, const void* diag, const void* b, void* x, int has_x0,
                     double tol_eff, double atol_eff, int restart, int64_t maxiter, int method, bk_result* result,
                     void* stream);
+/* ---- multicolor symmetric Gauss-Seidel preconditioner (AMGX's MULTICOLOR_GS, one symmetric sweep) -------------
+ * No reference counterpart: what users of the reference write as a callable M, kept on the device.
+ * bk_sgs_create colors A's pattern deterministically (Jones-Plassmann rounds over the neighbours j != i with (i, j) or
+ *   (j, i) stored, priority (fmix32(i) << 32) | i, smallest color no earlier-colored neighbour holds) and groups the rows
+ *   by color.  Every row must store a nonzero diagonal (the sum of its col == row entries): otherwise BK_ERR_ARG, naming
+ *   the row.  More than 255 colors: BK_ERR_UNSUPPORTED.  The result is cached, owned by A and freed with it.
+ * bk_sgs_get_info: the number of colors C and of coloring rounds.  bk_sgs_colors: the colors, copied to a device
+ *   uint8[n].
+ * bk_sgs_apply: z = M r with z = 0, a forward sweep over colors 0..C-1 and a backward sweep over C-2..0, every row
+ *   z_i = (r_i - sum_{j != i} a_ij z_j) / a_ii summed in CSR order (2C-1 kernels; bitwise reproducible).  The sweeps
+ *   read A's rowptr / col / val at every call, so an in-place update of the (borrowed) values is picked up by the next
+ *   application; only the coloring depends on the pattern.  (bk_*_jacobi, by contrast, take the diagonal the caller
+ *   extracted.)  r and z must not alias.
+ * bk_cg_sgs / bk_bicgstab_sgs / bk_gmres_sgs: arguments, recurrences and result fields of bk_cg_jacobi /
+ *   bk_bicgstab_jacobi / bk_gmres_jacobi with M = bk_sgs_apply.  A_sys may differ from the matrix S was built from
+ *   (same order and dtype): the adjoint solve runs on A^T with the M of A. */
+int bk_sgs_create(bk_handle* h, bk_csr* A, void* stream, bk_sgs** out);
+int bk_sgs_get_info(const bk_sgs* S, int32_t* ncolors, int32_t* rounds);
+int bk_sgs_colors(const bk_sgs* S, void* out, void* stream);
+int bk_sgs_apply(bk_handle* h, const bk_sgs* S, const void* r, void* z, void* stream);
+int bk_cg_sgs(bk_handle* h, const bk_csr* A_sys, const bk_sgs* S, const void* b, void* x, int has_x0, double tol,
+              double atol, int64_t maxiter, bk_result* result, void* stream);
+int bk_bicgstab_sgs(bk_handle* h, const bk_csr* A_sys, const bk_sgs* S, const void* b, void* x, int has_x0, double tol,
+                    double atol, int64_t maxiter, bk_result* result, void* stream);
+int bk_gmres_sgs(bk_handle* h, const bk_csr* A_sys, const bk_sgs* S, const void* b, void* x, int has_x0,
+                 double tol_eff, double atol_eff, int restart, int64_t maxiter, int method, bk_result* result,
+                 void* stream);
 /* out[r] = A[r][r] (0 when the row stores no diagonal entry); out: device vector of A's dtype */
 int bk_csr_diagonal(bk_handle* h, const bk_csr* A, void* out, void* stream);
 /* bk_gmres replaces gmres :641-784, _gmres_solve_with_method :788-803, _gmres_batched :431-493,

@@ -105,14 +105,16 @@ struct bk_bicg_vecs {
   T *x, *r, *rhat, *p, *q, *s, *t;
   T *phat, *shat;  // Jacobi: the preconditioned copies the SpMVs gather from
   const T* d;      // Jacobi: diag(A); nullptr = unpreconditioned
+  const bk_sgs* S; // symmetric Gauss-Seidel: phat = M p, shat = M s by the sweeps (d unused)
 };
 
 template <typename T, typename Sys>
 static int bk_bicg_enqueue_iter(const Sys& sys, const bk_bicg_vecs<T>& v, cudaStream_t s) {
   bk_dev_state* st = sys.h->st;
-  const bool pc = v.d != nullptr;
-  const bool al = !pc || bk_aligned16(v.d);
-  if (pc) {
+  const bool jac = v.d != nullptr;
+  const bool pc = jac || v.S;
+  const bool al = !jac || bk_aligned16(v.d);
+  if (jac) {
     bk_op_bicg_p_pc<T> op;
     op.r = v.r;
     op.p = v.p;
@@ -128,9 +130,10 @@ static int bk_bicg_enqueue_iter(const Sys& sys, const bk_bicg_vecs<T>& v, cudaSt
     op.q = v.q;
     op.st = st;
     BK_TRY(sys.template ew<T>(op, true, 2, s));
+    if (v.S) BK_TRY(bk_sgs_run(sys.h, v.S, v.p, v.phat, 1, s));
   }
   BK_TRY((sys.template matvec<T, 0, 1>(pc ? v.phat : v.p, v.q, v.rhat, nullptr, 1, bk_epi_bicg_alpha<T>{st}, s)));
-  if (pc) {
+  if (jac) {
     bk_op_bicg_s_pc<T> op;
     op.r = v.r;
     op.q = v.q;
@@ -146,6 +149,7 @@ static int bk_bicg_enqueue_iter(const Sys& sys, const bk_bicg_vecs<T>& v, cudaSt
     op.s = v.s;
     op.st = st;
     BK_TRY(sys.template ew<T>(op, true, 1, s));
+    if (v.S) BK_TRY(bk_sgs_run(sys.h, v.S, v.s, v.shat, 3, s));
   }
   // t = A shat ; the dots are t.s and t.t with the UNpreconditioned s (:926-930)
   BK_TRY((sys.template matvec<T, 0, 3>(pc ? v.shat : v.s, v.t, v.s, nullptr, 3, bk_epi_bicg_omega<T>{st}, s)));
@@ -176,7 +180,8 @@ static int bk_bicg_enqueue_iter(const Sys& sys, const bk_bicg_vecs<T>& v, cudaSt
 
 template <typename T, typename Sys>
 static int bk_bicgstab_t(const Sys& sys, const void* b, void* x_user, int has_x0, double tol, double atol,
-                         int64_t maxiter, bk_result* res, cudaStream_t s, const T* diag = nullptr) {
+                         int64_t maxiter, bk_result* res, cudaStream_t s, const T* diag = nullptr,
+                         const bk_sgs* S = nullptr) {
   bk_handle* h = sys.h;
   const long long n = sys.n();
   const size_t npad = ((size_t)n + 63) & ~(size_t)63;
@@ -192,6 +197,7 @@ static int bk_bicgstab_t(const Sys& sys, const void* b, void* x_user, int has_x0
   v.phat = v.t + npad;
   v.shat = v.phat + npad;
   v.d = diag;
+  v.S = S;
   bk_dev_state* st = h->st;
   const size_t vbytes = (size_t)n * sizeof(T);
   bk_call_begin(h, s, "bk_bicgstab");
@@ -218,13 +224,15 @@ static int bk_bicgstab_t(const Sys& sys, const void* b, void* x_user, int has_x0
   BK_CUDA(cudaMemcpyAsync(v.p, v.r, vbytes, cudaMemcpyDeviceToDevice, s));
   BK_CUDA(cudaMemcpyAsync(v.q, v.r, vbytes, cudaMemcpyDeviceToDevice, s));
 
-  const double bytes_iter = 2.0 * sys.matrix_bytes() + (diag ? 25.0 : 19.0) * n * sizeof(T);
-  const int chunk = bk_pick_chunk(h, bytes_iter, 5);
+  const int kernels_iter = 5 + (S ? 2 * bk_sgs_launches(S) : 0);
+  const double bytes_iter = (S ? 6.0 : 2.0) * sys.matrix_bytes() + (diag || S ? 25.0 : 19.0) * n * sizeof(T);
+  const int chunk = bk_pick_chunk(h, bytes_iter, kernels_iter);
   const bool use_graph = h->loop_mode != BK_LOOP_STREAM;
   uint64_t key[6] = {2 /*bicgstab*/, sys.uid(), (uint64_t)(uintptr_t)h->ws, (uint64_t)n,
                      (uint64_t)sys.dtype() | ((uint64_t)chunk << 16),
                      (uint64_t)bk_grid_spmv(h) | ((uint64_t)bk_grid_vec(h) << 32)};
   if (diag) key[1] ^= (uint64_t)(uintptr_t)diag * 0x9e3779b97f4a7c15ull;  // its address is baked into the graph
+  if (S) key[1] ^= (uint64_t)(uintptr_t)S * 0xc2b2ae3d27d4eb4full;
   auto enqueue_chunk = [&](cudaStream_t cs) -> int {
     for (int it = 0; it < chunk; ++it) BK_TRY((bk_bicg_enqueue_iter<T, Sys>(sys, v, cs)));
     return BK_OK;
@@ -236,7 +244,7 @@ static int bk_bicgstab_t(const Sys& sys, const void* b, void* x_user, int has_x0
     // launch-bound (L2-resident) systems: the whole loop in ONE persistent kernel (bk_bicgstab_persist.cuh);
     // phat / shat (unused without a preconditioner) serve as the second p / q buffers
     const bk_csr* A = sys.A;
-    if (diag == nullptr && A->rowptr && A->col) {
+    if (diag == nullptr && S == nullptr && A->rowptr && A->col) {
       bk_bp_args ga;
       ga.rowptr = A->rowptr;
       ga.col = A->col;
@@ -268,6 +276,10 @@ static int bk_bicgstab_t(const Sys& sys, const void* b, void* x_user, int has_x0
     op.epi = bk_epi_final_r2{st};
     BK_TRY(sys.template ew<T>(op, bk_aligned16(diag), 1, s));
   }
+  if (S) {
+    BK_TRY(bk_sgs_run(h, S, v.t, v.phat, 0, s));
+    BK_TRY((sys.template dot<T>(v.phat, v.phat, bk_epi_final_r2{st}, 1, s)));
+  }
   BK_TRY((sys.template dot<T>(v.x, v.x, bk_epi_final_x2{st}, 1, s)));
   BK_CUDA(cudaMemcpyAsync(x_user, v.x, vbytes, cudaMemcpyDeviceToDevice, s));
   BK_CUDA(cudaMemcpyAsync(&h->st_host[3], st, sizeof(bk_dev_state), cudaMemcpyDeviceToHost, s));
@@ -276,7 +288,8 @@ static int bk_bicgstab_t(const Sys& sys, const void* b, void* x_user, int has_x0
   const bk_dev_state* fin = &h->st_host[3];
   bk_fill_result_isolve(fin, res, 2 * fin->k + (has_x0 ? 1 : 0));
   res->rr_last = fin->rs;
-  res->kernel_launches = (persistent ? 1 : chunks * chunk * 5) + 2 + (has_x0 ? 1 : 0) + 2;
+  res->kernel_launches = (persistent ? 1 : chunks * chunk * kernels_iter) + 2 + (has_x0 ? 1 : 0) + 2 +
+                         (S ? bk_sgs_launches(S) + 1 : 0);
   bk_call_finish(h, res);
   return sys.check_comm(fin, "bicgstab");
 }
@@ -306,6 +319,20 @@ extern "C" int bk_bicgstab_jacobi(bk_handle* h, const bk_csr* A, const void* dia
                                  (const double*)diag);
   return bk_bicgstab_t<float>(sys, b, x, has_x0, tol, atol, maxiter, result, (cudaStream_t)stream,
                               (const float*)diag);
+}
+
+/* BiCGStab with the built-in symmetric Gauss-Seidel preconditioner: the right preconditioning of bk_bicgstab_jacobi
+ * with phat = M p and shat = M s computed by the sweeps. */
+extern "C" int bk_bicgstab_sgs(bk_handle* h, const bk_csr* A, const bk_sgs* S, const void* b, void* x, int has_x0,
+                               double tol, double atol, int64_t maxiter, bk_result* result, void* stream) {
+  BK_TRY(bk_solver_args_check("bk_bicgstab_sgs", h, A, b, x, result));
+  BK_TRY(bk_sgs_args_check("bk_bicgstab_sgs", h, A, S));
+  BK_CUDA(cudaSetDevice(h->device));
+  if (A->n == 0) return BK_OK;
+  const bk_sys_local sys{h, A};
+  if (A->dtype == BK_F64)
+    return bk_bicgstab_t<double>(sys, b, x, has_x0, tol, atol, maxiter, result, (cudaStream_t)stream, nullptr, S);
+  return bk_bicgstab_t<float>(sys, b, x, has_x0, tol, atol, maxiter, result, (cudaStream_t)stream, nullptr, S);
 }
 
 // Row-partitioned BiCGStab: same driver, every reduction made global (SURVEY §8e: "BiCGStab: 3 allreduce points").

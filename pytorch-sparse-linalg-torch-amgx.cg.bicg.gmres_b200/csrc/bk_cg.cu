@@ -428,21 +428,50 @@ struct bk_epi_pcg_bs {  // bs = b.b ; atol2 (:815-817)
 struct bk_epi_ignore {
   __device__ __forceinline__ void operator()(const double*) const {}
 };
+// Symmetric Gauss-Seidel CG (M = bk_sgs_run, z stored): K2 is the unpreconditioned bk_op_cg_r (r -= alpha Ap and the
+// stop test on r.r, which it leaves in gamma); the r.z reduction after the sweeps then sets beta = r.z / rho and puts r.z
+// into both rho and gamma, so the next SpMV's epilogue forms alpha = r.z / p.Ap.
+struct bk_epi_sgs_rr0 {  // first stop test on r0.r0 (:841) — atol2 was set by the b.b reduction
+  bk_dev_state* st;
+  __device__ __forceinline__ void operator()(const double* s) const {
+    st->rs = s[0];
+    if (st->maxiter <= 0) {
+      st->done = 1;
+      st->status = BK_ST_MAXITER;
+    }
+    if (s[0] <= st->atol2) {
+      st->done = 1;
+      st->status = BK_ST_CONVERGED;
+    }
+  }
+};
+struct bk_epi_sgs_rz {  // init: gamma = r0.z0 ; in the loop: beta = r.z / rho, gamma = r.z   (:826, :850-851)
+  bk_dev_state* st;
+  int init;
+  __device__ __forceinline__ void operator()(const double* s) const {
+    if (!init) st->beta = s[0] / st->rho;
+    st->rho = s[0];
+    st->gamma = s[0];
+  }
+};
 
+// Preconditioned CG.  M is either Jacobi (d = diag(A), S = nullptr: z = r / d formed on the fly inside the BLAS-1
+// kernels) or symmetric Gauss-Seidel (S != nullptr, d unused: z = M r stored by the sweeps).
 template <typename T, typename Sys>
 static int bk_pcg_t(const Sys& sys, const T* d, const void* b, void* x_user, int has_x0, double tol,
-                    double atol, int64_t maxiter, bk_result* res, cudaStream_t s) {
+                    double atol, int64_t maxiter, bk_result* res, cudaStream_t s, const bk_sgs* S = nullptr) {
   bk_handle* h = sys.h;
   const long long n = sys.n();
   const size_t npad = ((size_t)n + 63) & ~(size_t)63;
-  BK_TRY(bk_ws_reserve(h, (size_t)4 * npad * sizeof(T)));
+  BK_TRY(bk_ws_reserve(h, (size_t)(S ? 5 : 4) * npad * sizeof(T)));
   T* x = (T*)h->ws;
   T* r = x + npad;
   T* p = r + npad;
   T* ap = p + npad;
+  T* z = ap + npad;  // SGS only
   bk_dev_state* st = h->st;
   const size_t vbytes = (size_t)n * sizeof(T);
-  bk_call_begin(h, s, "bk_cg_jacobi");
+  bk_call_begin(h, s, S ? "bk_cg_sgs" : "bk_cg_jacobi");
 
   bk_dev_state init;
   memset(&init, 0, sizeof(init));
@@ -460,7 +489,12 @@ static int bk_pcg_t(const Sys& sys, const T* d, const void* b, void* x_user, int
     BK_CUDA(cudaMemsetAsync(x, 0, vbytes, s));
     BK_CUDA(cudaMemcpyAsync(r, b, vbytes, cudaMemcpyDeviceToDevice, s));
   }
-  {
+  if (S) {  // z0 = M r0 ; p0 = z0 ; rho = r0.z0 ; the stop test on r0.r0
+    BK_TRY(bk_sgs_run(h, S, r, z, 0, s));
+    BK_CUDA(cudaMemcpyAsync(p, z, vbytes, cudaMemcpyDeviceToDevice, s));
+    BK_TRY((sys.template dot<T>(r, r, bk_epi_sgs_rr0{st}, 1, s)));
+    BK_TRY((sys.template dot<T>(r, z, bk_epi_sgs_rz{st, 1}, 1, s)));
+  } else {
     bk_op_pcg_init<T> op;
     op.r = r;
     op.d = d;
@@ -468,9 +502,33 @@ static int bk_pcg_t(const Sys& sys, const T* d, const void* b, void* x_user, int
     op.st = st;
     BK_TRY(sys.template ew<T>(op, bk_aligned16(d), 1, s));
   }
-  const bool al = bk_aligned16(d);
+  const bool al = S ? true : bk_aligned16(d);
   auto enqueue_iter = [&](cudaStream_t cs) -> int {
     BK_TRY((sys.template matvec<T, 0, 1>(p, ap, p, nullptr, 1, bk_epi_cg_pAp{st}, cs)));
+    if (S) {
+      bk_op_cg_r<T> opr;
+      opr.ap = ap;
+      opr.r = r;
+      opr.st = st;
+      opr.snake = 0;
+      BK_TRY(sys.template ew<T>(opr, true, 1, cs));
+      BK_TRY(bk_sgs_run(h, S, r, z, 1, cs));
+      bk_op_dot_epi<T, bk_epi_sgs_rz> opd;  // gamma = r.z in the fixed order of the grid reduction
+      opd.x = r;
+      opd.y = z;
+      opd.epi = bk_epi_sgs_rz{st, 0};
+      opd.st = st;
+      opd.guard = 1;
+      BK_TRY(sys.template ew<T>(opd, true, 1, cs));
+      bk_op_cg_xp<T> opx;  // x += alpha p ; p = z + beta p
+      opx.x = x;
+      opx.p = p;
+      opx.r = z;
+      opx.st = st;
+      opx.snake = 0;
+      BK_TRY(sys.template ew<T>(opx, true, 2, cs));
+      return BK_OK;
+    }
     {
       bk_op_pcg_r<T> op;
       op.ap = ap;
@@ -490,14 +548,15 @@ static int bk_pcg_t(const Sys& sys, const T* d, const void* b, void* x_user, int
     }
     return BK_OK;
   };
-  const double bytes_iter = sys.matrix_bytes() + 13.0 * n * sizeof(T);
-  const int chunk = bk_pick_chunk(h, bytes_iter, 3);
+  const int kernels_iter = S ? 4 + bk_sgs_launches(S) : 3;
+  const double bytes_iter = (S ? 3.0 : 1.0) * sys.matrix_bytes() + 13.0 * n * sizeof(T);
+  const int chunk = bk_pick_chunk(h, bytes_iter, kernels_iter);
   const bool use_graph = h->loop_mode != BK_LOOP_STREAM;
-  uint64_t key[6] = {5 /*jacobi cg*/, sys.uid(), (uint64_t)(uintptr_t)h->ws, (uint64_t)n,
+  uint64_t key[6] = {S ? 6ull /*sgs cg*/ : 5ull /*jacobi cg*/, sys.uid(), (uint64_t)(uintptr_t)h->ws, (uint64_t)n,
                      (uint64_t)sys.dtype() | ((uint64_t)chunk << 16) | ((uint64_t)al << 8),
                      (uint64_t)bk_grid_spmv(h) | ((uint64_t)bk_grid_vec(h) << 32)};
   // the diagonal's address is baked into the captured graph: make it part of the key
-  key[1] ^= (uint64_t)(uintptr_t)d * 0x9e3779b97f4a7c15ull;
+  key[1] ^= (uint64_t)(uintptr_t)(S ? (const void*)S : (const void*)d) * 0x9e3779b97f4a7c15ull;
   auto enqueue_chunk = [&](cudaStream_t cs) -> int {
     for (int it = 0; it < chunk; ++it) BK_TRY(enqueue_iter(cs));
     return BK_OK;
@@ -509,7 +568,10 @@ static int bk_pcg_t(const Sys& sys, const T* d, const void* b, void* x_user, int
 
   // final check of _isolve: || M (b - A x) || against max(tol ||b||, atol) (:1008-1013)
   BK_TRY((sys.template matvec<T, 1, 2>(x, ap, nullptr, b, 0, bk_epi_ignore{}, s)));
-  {
+  if (S) {
+    BK_TRY(bk_sgs_run(h, S, ap, z, 0, s));
+    BK_TRY((sys.template dot<T>(z, z, bk_epi_final_r{st}, 1, s)));
+  } else {
     bk_op_scaled_sq<T, bk_epi_final_r> op;
     op.t = ap;
     op.d = d;
@@ -523,10 +585,15 @@ static int bk_pcg_t(const Sys& sys, const T* d, const void* b, void* x_user, int
   BK_CUDA(cudaStreamSynchronize(s));
   const bk_dev_state* fin = &h->st_host[3];
   bk_fill_result_isolve(fin, res, fin->k + (has_x0 ? 1 : 0));
-  res->rr_last = fin->rs;
-  res->kernel_launches = chunks * chunk * 3 + 4 + (has_x0 ? 1 : 0) + 3;
+  if (S) {
+    res->rr_last = fin->k > 0 ? fin->gamma : fin->rs;  // the loop's last K2 left r.r in gamma
+    res->kernel_launches = chunks * chunk * kernels_iter + 4 + (has_x0 ? 1 : 0) + 2 * bk_sgs_launches(S) + 3;
+  } else {
+    res->rr_last = fin->rs;
+    res->kernel_launches = chunks * chunk * 3 + 4 + (has_x0 ? 1 : 0) + 3;
+  }
   bk_call_finish(h, res);
-  return sys.check_comm(fin, "cg_jacobi");
+  return sys.check_comm(fin, S ? "cg_sgs" : "cg_jacobi");
 }
 
 extern "C" int bk_cg_jacobi(bk_handle* h, const bk_csr* A, const void* diag, const void* b, void* x, int has_x0,
@@ -539,6 +606,18 @@ extern "C" int bk_cg_jacobi(bk_handle* h, const bk_csr* A, const void* diag, con
   if (A->dtype == BK_F64)
     return bk_pcg_t<double>(sys, (const double*)diag, b, x, has_x0, tol, atol, maxiter, result, (cudaStream_t)stream);
   return bk_pcg_t<float>(sys, (const float*)diag, b, x, has_x0, tol, atol, maxiter, result, (cudaStream_t)stream);
+}
+
+extern "C" int bk_cg_sgs(bk_handle* h, const bk_csr* A, const bk_sgs* S, const void* b, void* x, int has_x0,
+                         double tol, double atol, int64_t maxiter, bk_result* result, void* stream) {
+  BK_TRY(bk_solver_args_check("bk_cg_sgs", h, A, b, x, result));
+  BK_TRY(bk_sgs_args_check("bk_cg_sgs", h, A, S));
+  BK_CUDA(cudaSetDevice(h->device));
+  if (A->n == 0) return BK_OK;
+  const bk_sys_local sys{h, A};
+  if (A->dtype == BK_F64)
+    return bk_pcg_t<double>(sys, nullptr, b, x, has_x0, tol, atol, maxiter, result, (cudaStream_t)stream, S);
+  return bk_pcg_t<float>(sys, nullptr, b, x, has_x0, tol, atol, maxiter, result, (cudaStream_t)stream, S);
 }
 
 // diag[r] = A[r][r] (sum of the stored entries with col == r; 0 when the row has none)

@@ -1379,6 +1379,7 @@ extern "C" int bk_csr_destroy(bk_csr* A) {
     cudaDeviceSynchronize();  // nothing may still be reading the arrays: the frees below are stream-ordered
   }
   if (A->transpose) bk_csr_destroy(A->transpose);
+  if (A->sgs) bk_sgs_free(A->sgs);
   if (A->split) bk_csr_destroy(A->split);
   if (A->vstart) bk_pool_free(A->vstart);
   if (A->yv) bk_pool_free(A->yv);

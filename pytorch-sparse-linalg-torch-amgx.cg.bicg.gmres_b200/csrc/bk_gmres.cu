@@ -393,16 +393,17 @@ __global__ void bk_gm_solve_kernel(bk_dev_state* st, const bk_gm_small sm) {
 template <typename T, typename Sys>
 static int bk_gmres_t(const Sys& sys, const void* b, void* x_user, int has_x0, double tol_eff, double atol_eff,
                       int restart, int64_t maxiter, int method, bk_result* res, cudaStream_t s,
-                      const T* diag = nullptr) {
+                      const T* diag = nullptr, const bk_sgs* S = nullptr) {
   bk_handle* h = sys.h;
   const long long n = sys.n();
   const int m = restart;
   const size_t npad = ((size_t)n + 63) & ~(size_t)63;
-  BK_TRY(bk_ws_reserve(h, (size_t)(m + 4) * npad * sizeof(T)));
+  BK_TRY(bk_ws_reserve(h, (size_t)(m + (S ? 5 : 4)) * npad * sizeof(T)));
   T* V = (T*)h->ws;
   T* w = V + (size_t)(m + 1) * npad;
   T* x = w + npad;
   T* bw = x + npad;  // private copy of b: keeps the cached cycle graph independent of the caller's pointer
+  T* u = bw + npad;  // SGS: the A-product the sweeps read (they cannot work in place)
   bk_dev_state* st = h->st;
   const size_t vbytes = (size_t)n * sizeof(T);
   constexpr int NW = bk_native_w<T>::value;
@@ -487,21 +488,38 @@ static int bk_gmres_t(const Sys& sys, const void* b, void* x_user, int has_x0, d
     op.guard = guard;
     return sys.template ew<T>(op, dal, 1, cs);
   };
+  // left symmetric Gauss-Seidel preconditioning (S != nullptr): the A-product goes to u, the sweeps write w = M u and
+  // a guarded reduction carries the norm
+  auto sgs_sq = [&](const T* src, auto epi, int guard, cudaStream_t cs) -> int {
+    BK_TRY(bk_sgs_run(h, S, src, w, guard, cs));
+    bk_op_dot_epi<T, decltype(epi)> op;
+    op.x = w;
+    op.y = w;
+    op.epi = epi;
+    op.st = st;
+    op.guard = guard;
+    return sys.template ew<T>(op, true, 1, cs);
+  };
   if (diag) {
     BK_CUDA(cudaMemcpyAsync(w, b, vbytes, cudaMemcpyDeviceToDevice, s));
     BK_TRY(scale_sq(w, bk_epi_gm_ptol{st}, 0, s));  // w = M b (also r0 when x0 = 0)
+  } else if (S) {
+    BK_TRY(sgs_sq((const T*)b, bk_epi_gm_ptol{st}, 0, s));
   }
   if (has_x0) {
     BK_CUDA(cudaMemcpyAsync(x, x_user, vbytes, cudaMemcpyDeviceToDevice, s));
     if (diag) {
       BK_TRY((sys.template matvec<T, 1, 2>(x, w, nullptr, b, 0, bk_epi_gm_ignore{}, s)));
       BK_TRY(scale_sq(w, bk_epi_gm_resid<T>{st, sm, 1}, 0, s));
+    } else if (S) {
+      BK_TRY((sys.template matvec<T, 1, 2>(x, u, nullptr, b, 0, bk_epi_gm_ignore{}, s)));
+      BK_TRY(sgs_sq(u, bk_epi_gm_resid<T>{st, sm, 1}, 0, s));
     } else {
       BK_TRY((sys.template matvec<T, 1, 2>(x, w, nullptr, b, 0, bk_epi_gm_resid<T>{st, sm, 1}, s)));
     }
   } else {
     BK_CUDA(cudaMemsetAsync(x, 0, vbytes, s));
-    if (diag) {  // w already holds M b; its norm is ||M b|| = sqrt of what the ptol pass summed: recompute cheaply
+    if (diag || S) {  // w already holds M b; its norm is ||M b|| = sqrt of what the ptol pass summed: recompute cheaply
       BK_TRY((sys.template dot<T>(w, w, bk_epi_gm_resid0<T>{st, sm}, 1, s)));
     } else {
       BK_CUDA(cudaMemcpyAsync(w, b, vbytes, cudaMemcpyDeviceToDevice, s));
@@ -517,6 +535,9 @@ static int bk_gmres_t(const Sys& sys, const void* b, void* x_user, int has_x0, d
       if (diag) {
         BK_TRY((sys.template matvec<T, 0, 2>(V + (size_t)j * npad, w, nullptr, nullptr, 2, bk_epi_gm_ignore{}, cs)));
         BK_TRY(scale_sq(w, bk_epi_gm_vnorm0<T>{st}, 2, cs));
+      } else if (S) {
+        BK_TRY((sys.template matvec<T, 0, 2>(V + (size_t)j * npad, u, nullptr, nullptr, 2, bk_epi_gm_ignore{}, cs)));
+        BK_TRY(sgs_sq(u, bk_epi_gm_vnorm0<T>{st}, 2, cs));
       } else {
         BK_TRY((sys.template matvec<T, 0, 2>(V + (size_t)j * npad, w, nullptr, nullptr, 2, bk_epi_gm_vnorm0<T>{st}, cs)));
       }
@@ -540,6 +561,9 @@ static int bk_gmres_t(const Sys& sys, const void* b, void* x_user, int has_x0, d
     if (diag) {
       BK_TRY((sys.template matvec<T, 1, 2>(x, w, nullptr, b, 1, bk_epi_gm_ignore{}, cs)));
       BK_TRY(scale_sq(w, bk_epi_gm_resid<T>{st, sm, 0}, 1, cs));
+    } else if (S) {
+      BK_TRY((sys.template matvec<T, 1, 2>(x, u, nullptr, b, 1, bk_epi_gm_ignore{}, cs)));
+      BK_TRY(sgs_sq(u, bk_epi_gm_resid<T>{st, sm, 0}, 1, cs));
     } else {
       BK_TRY((sys.template matvec<T, 1, 2>(x, w, nullptr, b, 1, bk_epi_gm_resid<T>{st, sm, 0}, cs)));
     }
@@ -551,13 +575,14 @@ static int bk_gmres_t(const Sys& sys, const void* b, void* x_user, int has_x0, d
                      (uint64_t)sys.dtype() | ((uint64_t)m << 8) | ((uint64_t)method << 24),
                      (uint64_t)bk_grid_spmv(h) | ((uint64_t)bk_grid_vec(h) << 32)};
   if (diag) key[1] ^= (uint64_t)(uintptr_t)diag * 0x9e3779b97f4a7c15ull;  // its address is baked into the graph
+  if (S) key[1] ^= (uint64_t)(uintptr_t)S * 0xc2b2ae3d27d4eb4full;
   int64_t chunks = 0;
   bk_call_mark(h, "loop");
   bool persistent = false;
   if constexpr (!Sys::kDist) {
     // launch-bound (L2-resident) systems: the whole solve in ONE cooperative kernel (bk_gmres_persist.cuh)
     const bk_csr* A = sys.A;
-    if (A->rowptr && A->col) {
+    if (S == nullptr && A->rowptr && A->col) {
       bk_gp_args ga;
       ga.rowptr = A->rowptr;
       ga.col = A->col;
@@ -592,6 +617,8 @@ static int bk_gmres_t(const Sys& sys, const void* b, void* x_user, int has_x0, d
   res->iterations = fin->k;
   res->matvecs = fin->matvecs;
   res->kernel_launches = (persistent ? 1 : chunks * (4 * (int64_t)m + 4)) + 5;
+  if (S)  // every A-product is followed by the sweeps and the norm: m + 1 per cycle, 2 (3 with x0) in the set-up
+    res->kernel_launches += (chunks * (m + 1) + 2 + (has_x0 ? 1 : 0)) * (int64_t)(bk_sgs_launches(S) + 1);
   res->status = fin->status;
   res->final_residual = sqrt(fmax(fin->rtrue2, 0.0));
   res->b_norm = fin->g_bnorm;
@@ -601,6 +628,26 @@ static int bk_gmres_t(const Sys& sys, const void* b, void* x_user, int has_x0, d
   const bool failed = (res->x_norm != res->x_norm) || (res->final_residual > res->threshold);
   res->info = failed ? -1 : 0;
   return sys.check_comm(fin, "gmres");
+}
+
+static int bk_gmres_args_check(const char* who, int restart, int method);
+
+/* GMRES with the built-in symmetric Gauss-Seidel preconditioner applied from the left (v = M(A v), r = M(b - A x),
+ * ptol from ||M b||, final check on ||M(b - A x)||), as bk_gmres_jacobi. */
+extern "C" int bk_gmres_sgs(bk_handle* h, const bk_csr* A, const bk_sgs* S, const void* b, void* x, int has_x0,
+                            double tol_eff, double atol_eff, int restart, int64_t maxiter, int method, bk_result* result,
+                            void* stream) {
+  BK_TRY(bk_solver_args_check("bk_gmres_sgs", h, A, b, x, result));
+  BK_TRY(bk_gmres_args_check("bk_gmres_sgs", restart, method));
+  BK_TRY(bk_sgs_args_check("bk_gmres_sgs", h, A, S));
+  BK_CUDA(cudaSetDevice(h->device));
+  if (A->n == 0) return BK_OK;
+  const bk_sys_local sys{h, A};
+  if (A->dtype == BK_F64)
+    return bk_gmres_t<double>(sys, b, x, has_x0, tol_eff, atol_eff, restart, maxiter, method, result,
+                              (cudaStream_t)stream, nullptr, S);
+  return bk_gmres_t<float>(sys, b, x, has_x0, tol_eff, atol_eff, restart, maxiter, method, result,
+                           (cudaStream_t)stream, nullptr, S);
 }
 
 static int bk_gmres_args_check(const char* who, int restart, int method) {

@@ -141,6 +141,7 @@ struct bk_csr {
   int max_row_nnz;
   double mean_row_nnz;
   bk_csr* transpose;  // cached, owned
+  bk_sgs* sgs;        // multicolor symmetric Gauss-Seidel set-up (bk_sgs_create), cached, owned
   // long-row splitting (skewed matrices): `split` views the same col/val arrays through a finer row pointer in which
   // every row longer than BK_SPLIT_LEN is cut into virtual rows; vstart[r] = first virtual row of real row r
   bk_csr* split;      // owned (its rowptr only)
@@ -149,6 +150,23 @@ struct bk_csr {
   int is_view;        // this object borrows col/val/tails from a parent (do not free them)
   uint64_t uid;       // unique id for graph-cache keys
 };
+
+// multicolor symmetric Gauss-Seidel (bk_sgs.cu): the coloring of A's pattern and its rows grouped by color.  The
+// sweeps read rowptr / col / val of `A` at every application, so an in-place update of the values is picked up.
+struct bk_sgs {
+  const bk_csr* A;
+  int ncolors, rounds;
+  unsigned char* colors;  // [n], own
+  int* rows;              // [n] rows sorted by color (stable: ascending within a color), own
+  int* offs;              // host [ncolors + 1]: rows of color c are rows[offs[c] .. offs[c+1])
+};
+void bk_sgs_free(bk_sgs* S);
+// z = M r: the forward sweep over colors 0..C-1, then the backward sweep over C-2..0 (2C-1 kernels).  Every kernel
+// returns at once when bk_guard_skip(st, guard) holds.  r and z must not alias.
+int bk_sgs_run(bk_handle* h, const bk_sgs* S, const void* r, void* z, int guard, cudaStream_t s);
+static inline int bk_sgs_launches(const bk_sgs* S) { return 2 * S->ncolors - 1; }
+// the checks every bk_*_sgs entry shares: S belongs to h and fits A_sys (order, dtype)
+int bk_sgs_args_check(const char* who, bk_handle* h, const bk_csr* A, const bk_sgs* S);
 
 // ------------------------------------------------------------------------------------------
 // handle

@@ -21,6 +21,7 @@ _LIB_DIR = Path(__file__).resolve().parent / "_lib"
 BK_F64, BK_F32 = 0, 1
 BK_GMRES_BATCHED, BK_GMRES_INCREMENTAL = 0, 1
 METHOD_CG, METHOD_BICGSTAB, METHOD_GMRES = 0, 1, 2
+BK_ERR_ARG = -1
 
 
 class NativeLibraryError(RuntimeError):
@@ -124,6 +125,16 @@ _SIGNATURES = {
     "bk_gmres_jacobi": (C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int64,
                                   C.c_int, C.POINTER(bk_result), _VP]),
     "bk_csr_diagonal": (C.c_int, [_VP, _VP, _VP, _VP]),
+    "bk_sgs_create": (C.c_int, [_VP, _VP, _VP, C.POINTER(_VP)]),
+    "bk_sgs_get_info": (C.c_int, [_VP, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
+    "bk_sgs_colors": (C.c_int, [_VP, _VP, _VP]),
+    "bk_sgs_apply": (C.c_int, [_VP, _VP, _VP, _VP, _VP]),
+    "bk_cg_sgs": (C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int, C.c_double, C.c_double, C.c_int64,
+                            C.POINTER(bk_result), _VP]),
+    "bk_bicgstab_sgs": (C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int, C.c_double, C.c_double, C.c_int64,
+                                  C.POINTER(bk_result), _VP]),
+    "bk_gmres_sgs": (C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int64,
+                               C.c_int, C.POINTER(bk_result), _VP]),
     "bk_dist_bicgstab": (C.c_int, [_VP, _VP, _VP, _VP, C.c_int, C.c_double, C.c_double, C.c_int64, C.c_int64,
                                    C.POINTER(bk_result), _VP]),
     "bk_dist_gmres": (C.c_int, [_VP, _VP, _VP, _VP, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int64, C.c_int,
@@ -258,6 +269,7 @@ class CsrMatrix:
         self.ptr = p
         self._owned = True
         self._transpose = None
+        self._sgs = None
         self._finalizer = weakref.finalize(self, CsrMatrix._destroy, handle.lib, p)
 
     @staticmethod
@@ -274,6 +286,7 @@ class CsrMatrix:
         obj._keep = keep
         obj._owned = False
         obj._transpose = None
+        obj._sgs = None
         return obj
 
     def info(self) -> dict:
@@ -290,6 +303,20 @@ class CsrMatrix:
                                                         C.byref(p)), "bk_csr_transpose")
             self._transpose = CsrMatrix._wrap(self.handle, p, self.n, self.nnz, self.dtype, self.device, (self,))
         return self._transpose
+
+    def sgs(self) -> "SgsPreconditioner":
+        """Cached multicolor symmetric Gauss-Seidel set-up of this matrix (owned by it on the C side).
+        ValueError when a row stores no nonzero diagonal."""
+        if self._sgs is None:
+            p = _VP()
+            with torch.cuda.device(self.device):
+                rc = self.handle.lib.bk_sgs_create(self.handle.ptr, self.ptr, _stream_ptr(self.device), C.byref(p))
+            if rc == BK_ERR_ARG:
+                msg = self.handle.lib.bk_last_error()
+                raise ValueError(msg.decode() if msg else "bk_sgs_create: invalid matrix")
+            _check(rc, "bk_sgs_create")
+            self._sgs = SgsPreconditioner(self, p)
+        return self._sgs
 
     def arrays(self) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
         """Copy the (int32) CSR arrays of this matrix out as torch tensors (testing / debugging)."""
@@ -428,6 +455,63 @@ class CsrMatrix:
     def bicgstab_jacobi(self, diag: torch.Tensor, b, x0, tol, atol, maxiter):
         """BiCGStab right-preconditioned with M = (v -> v / diag), all on the device (bk_bicgstab_jacobi)."""
         return self._solve_jacobi("bk_bicgstab_jacobi", diag, b, x0, tol, atol, maxiter)
+
+    def _solve_sgs(self, fn_name: str, S: "SgsPreconditioner", b, x0, *args):
+        if S.n != self.n or S.dtype != self.dtype or S.device != self.device:
+            raise ValueError("the preconditioner was built for another order, dtype or device")
+        b = self._vec(b)
+        if x0 is None:
+            x, has_x0 = torch.empty_like(b), 0
+        else:
+            x, has_x0 = self._vec(x0).clone(), 1
+        res = bk_result()
+        with torch.cuda.device(self.device):
+            rc = getattr(self.handle.lib, fn_name)(self.handle.ptr, self.ptr, S.ptr, b.data_ptr(), x.data_ptr(),
+                                                   has_x0, *args, C.byref(res), _stream_ptr(self.device))
+        _check(rc, fn_name)
+        return x, res.as_dict()
+
+    def cg_sgs(self, S: "SgsPreconditioner", b, x0, tol, atol, maxiter):
+        """CG preconditioned with multicolor symmetric Gauss-Seidel, all on the device (bk_cg_sgs)."""
+        return self._solve_sgs("bk_cg_sgs", S, b, x0, float(tol), float(atol), -1 if maxiter is None else int(maxiter))
+
+    def bicgstab_sgs(self, S: "SgsPreconditioner", b, x0, tol, atol, maxiter):
+        """BiCGStab right-preconditioned with symmetric Gauss-Seidel (bk_bicgstab_sgs)."""
+        return self._solve_sgs("bk_bicgstab_sgs", S, b, x0, float(tol), float(atol),
+                               -1 if maxiter is None else int(maxiter))
+
+    def gmres_sgs(self, S: "SgsPreconditioner", b, x0, tol_eff, atol_eff, restart, maxiter, method):
+        """GMRES left-preconditioned with symmetric Gauss-Seidel (bk_gmres_sgs)."""
+        return self._solve_sgs("bk_gmres_sgs", S, b, x0, float(tol_eff), float(atol_eff), int(restart),
+                               -1 if maxiter is None else int(maxiter), int(method))
+
+
+class SgsPreconditioner:
+    """A bk_sgs of a registered matrix (freed with it; this object keeps the matrix alive)."""
+
+    def __init__(self, mat: CsrMatrix, ptr):
+        self.mat, self.ptr = mat, ptr
+        self.n, self.dtype, self.device = mat.n, mat.dtype, mat.device
+        nc, rounds = C.c_int32(), C.c_int32()
+        _check(mat.handle.lib.bk_sgs_get_info(ptr, C.byref(nc), C.byref(rounds)), "bk_sgs_get_info")
+        self.num_colors, self.rounds = nc.value, rounds.value
+
+    def colors(self) -> torch.Tensor:
+        """The color of every row (uint8, on the device)."""
+        out = torch.empty(self.n, dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            _check(self.mat.handle.lib.bk_sgs_colors(self.ptr, out.data_ptr(), _stream_ptr(self.device)),
+                   "bk_sgs_colors")
+        return out
+
+    def apply(self, r: torch.Tensor) -> torch.Tensor:
+        """z = M r (bk_sgs_apply)."""
+        r = self.mat._vec(r)
+        z = torch.empty_like(r)
+        with torch.cuda.device(self.device):
+            _check(self.mat.handle.lib.bk_sgs_apply(self.mat.handle.ptr, self.ptr, r.data_ptr(), z.data_ptr(),
+                                                    _stream_ptr(self.device)), "bk_sgs_apply")
+        return z
 
 
 # ---- building-block vector ops (deterministic reductions) ------------------------------------------

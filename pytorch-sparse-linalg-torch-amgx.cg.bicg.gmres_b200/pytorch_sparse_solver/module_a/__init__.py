@@ -5,7 +5,7 @@ from .krylov import (
     cg_differentiable, bicgstab_differentiable, gmres_differentiable,
     LinearSolveFunction,
 )
-from .preconditioners import BlockJacobiPreconditioner, JacobiPreconditioner
+from .preconditioners import BlockJacobiPreconditioner, JacobiPreconditioner, SymmetricGaussSeidelPreconditioner
 from .mixed_precision import refined_solve
 from .torch_tree_util import tree_leaves, tree_map, tree_flatten, tree_unflatten, Partial
 
@@ -15,6 +15,7 @@ __all__ = [
     'LinearSolveFunction',
     'JacobiPreconditioner',   # addition: built-in M that keeps cg() on the device (SURVEY §8f-1)
     'BlockJacobiPreconditioner',   # addition: block-diagonal M applied by one library kernel
+    'SymmetricGaussSeidelPreconditioner',   # addition: multicolor symmetric Gauss-Seidel M, on the device
     'refined_solve',          # addition: mixed-precision iterative refinement (SURVEY §8f-4)
     'tree_leaves', 'tree_map', 'tree_flatten', 'tree_unflatten', 'Partial',
 ]

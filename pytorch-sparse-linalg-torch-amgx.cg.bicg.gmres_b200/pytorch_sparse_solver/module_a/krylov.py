@@ -35,7 +35,7 @@ from typing import Any, Callable, Optional, Tuple, Union
 import torch
 
 from .. import _native
-from .preconditioners import JacobiPreconditioner
+from .preconditioners import JacobiPreconditioner, SymmetricGaussSeidelPreconditioner
 from .torch_tree_util import tree_leaves
 
 __all__ = [
@@ -88,11 +88,11 @@ def _check_x0(b, x0):
 
 
 def _route(A, b, x0, M, native_M: bool = False) -> str:
-    """native_M: the solver has a device implementation for a built-in preconditioner object (Jacobi)."""
+    """native_M: the solver has a device implementation for a built-in preconditioner object (Jacobi, SGS)."""
     kind = _check_operator(A)
     if kind == "tensor" and isinstance(b, torch.Tensor) and (A.is_complex() or b.is_complex()):
         return "complex"
-    builtin = native_M and isinstance(M, JacobiPreconditioner) and kind == "tensor" and A.is_cuda
+    builtin = native_M and isinstance(M, _BUILTIN_M) and kind == "tensor" and A.is_cuda
     if kind == "callable" or (M is not None and not builtin) or not isinstance(b, torch.Tensor):
         return "generic"
     if b.ndim != 1 or b.shape[0] != A.shape[0]:
@@ -102,6 +102,9 @@ def _route(A, b, x0, M, native_M: bool = False) -> str:
     if A.is_cuda != b.is_cuda:
         raise ValueError("A and b must live on the same device")
     return "native" if A.is_cuda else "host"
+
+
+_BUILTIN_M = (JacobiPreconditioner, SymmetricGaussSeidelPreconditioner)
 
 
 def _work_dtype(A: torch.Tensor, b: torch.Tensor) -> torch.dtype:
@@ -163,7 +166,14 @@ def _solve_core(name: str, A: torch.Tensor, b: torch.Tensor, x0: Optional[torch.
             mat = _native.register_matrix(A, wdt)
             if transpose:
                 mat = mat.transpose()
-            if name == "cg" and precond is not None:   # diag(A^T) == diag(A): the adjoint solve reuses M (:1079-1084)
+            sgs = precond.sgs(wdt) if isinstance(precond, SymmetricGaussSeidelPreconditioner) else None
+            if sgs is not None:   # the adjoint solve runs on A^T with the M of A, as the reference does with a callable M
+                if name == "gmres":
+                    tol_eff, atol_eff = _gmres_effective_tolerances(tol, atol, n, 'cuda')
+                    x, res = mat.gmres_sgs(sgs, bw, x0w, tol_eff, atol_eff, restart, maxiter, method)
+                else:
+                    x, res = getattr(mat, name + "_sgs")(sgs, bw, x0w, tol, atol, maxiter)
+            elif name == "cg" and precond is not None:   # diag(A^T) == diag(A): the adjoint solve reuses M (:1079-1084)
                 x, res = mat.cg_jacobi(precond.diagonal(wdt, bw.device), bw, x0w, tol, atol, maxiter)
             elif name == "cg":
                 x, res = mat.cg(bw, x0w, tol, atol, maxiter)

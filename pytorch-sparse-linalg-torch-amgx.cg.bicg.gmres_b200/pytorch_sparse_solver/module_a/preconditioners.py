@@ -6,6 +6,8 @@ what users of the reference write as `M = lambda r: r / d` — that `cg()`, `bic
 recognise: for a CUDA matrix the whole preconditioned iteration then stays on the device (`bk_cg_jacobi`,
 `bk_bicgstab_jacobi`, `bk_gmres_jacobi`), with results identical to passing the lambda to the reference (golden
 fixtures `*_jacobi*`).  With a callable `A` or on CPU tensors it behaves like any other callable `M`.
+`SymmetricGaussSeidelPreconditioner(A)` is the stronger built-in: one multicolor symmetric Gauss-Seidel sweep
+(`bk_cg_sgs`, `bk_bicgstab_sgs`, `bk_gmres_sgs` on the device route; a library call per application elsewhere).
 """
 from __future__ import annotations
 
@@ -106,3 +108,50 @@ class BlockJacobiPreconditioner:
         if inv is not self.inv:
             self.inv = inv
         return _native.block_apply(inv, r.detach(), self.bs).reshape(r.shape)
+
+
+class SymmetricGaussSeidelPreconditioner:
+    """M = one multicolor symmetric Gauss-Seidel sweep: z = 0, a forward sweep over the colors of A's pattern, then a
+    backward sweep, every row z_i = (r_i - sum_{j != i} a_ij z_j) / a_ii.  For symmetric A this is
+    M = (D + U)^-1 D (D + L)^-1 with the rows taken in color order, which is symmetric positive definite when A is.
+
+    The coloring (deterministic Jones-Plassmann rounds) is built once per work dtype, when A is first registered for it.
+    The sweeps read A's values at every application: when A is a CUDA CSR tensor of the work dtype, its values are
+    borrowed, so an in-place update of A.values() is picked up by the next application (JacobiPreconditioner, by
+    contrast, keeps the diagonal it read at construction).  Only a change of the sparsity pattern needs a new object.
+
+    cg(), bicgstab() and gmres() run the whole preconditioned iteration on the device with it (and reuse it for the
+    adjoint solve on A^T); as a callable `M(r)` it works on the generic route too, e.g. with a callable A."""
+
+    def __init__(self, A: torch.Tensor):
+        if type(A).__name__ == "DistMatrix":
+            raise ValueError("SymmetricGaussSeidelPreconditioner does not support row-partitioned matrices")
+        if not isinstance(A, torch.Tensor) or A.ndim != 2 or A.shape[0] != A.shape[1]:
+            raise ValueError("SymmetricGaussSeidelPreconditioner needs a square 2-D tensor (dense, COO or CSR)")
+        if A.is_complex():
+            raise ValueError("SymmetricGaussSeidelPreconditioner supports real matrices only")
+        if not A.is_cuda:
+            raise _native.NativeLibraryError("SymmetricGaussSeidelPreconditioner runs on the CUDA device "
+                                             "(no CPU fallback)")
+        self.A = A.detach()
+        self.shape = tuple(A.shape)
+        self._by_dtype = {}
+        self.sgs(torch.float32 if A.dtype == torch.float32 else torch.float64)   # checks the diagonal now
+
+    def sgs(self, dtype: torch.dtype) -> "_native.SgsPreconditioner":
+        """The device set-up for the work dtype `dtype` (registered and colored on first use, then cached)."""
+        S = self._by_dtype.get(dtype)
+        if S is None:
+            with torch.no_grad():
+                S = _native.register_matrix(self.A, dtype).sgs()
+            self._by_dtype[dtype] = S
+        return S
+
+    def __call__(self, r):
+        if not isinstance(r, torch.Tensor):
+            raise TypeError("SymmetricGaussSeidelPreconditioner applies to a single tensor")
+        if not r.is_cuda:
+            raise _native.NativeLibraryError("SymmetricGaussSeidelPreconditioner applies on the CUDA device "
+                                             "(no CPU fallback)")
+        wdt = torch.float32 if r.dtype == torch.float32 else torch.float64
+        return self.sgs(wdt).apply(r.detach().reshape(-1).to(wdt)).reshape(r.shape)
